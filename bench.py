@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...                                # the reference's CPU path (oracle port) on the host cores
     python bench.py --config c2|c4|c5 ...                               # the other BASELINE.json configurations (see CONFIGS)
+    python bench.py ... --dump-outputs DIR                              # also write what the last timed step computed, DIR/<name>.npy
 
 Headline step (c3, Multi-Task_Pretrain/models.py:306-335 + main_pretrain.py:701-832 for the encoder): three uint8 image streams
 (3 + 3 + 2 images per GPU) -> MTP_DataPreprocessor arithmetic fused into the patch gather -> ONE encoder call on the concatenated
@@ -21,6 +22,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 import torch  # noqa: E402
 
@@ -58,7 +60,14 @@ def parse():
     ap.add_argument("--comm-sms", type=int, default=16, help="SMs left to NCCL while the backward runs (N > 1)")
     ap.add_argument("--grad-comm", default="bf16", choices=["bf16", "fp32"], help="dtype of the gradient all-reduce buckets (N > 1)")
     ap.add_argument("--float-input", action="store_true", help="feed a pre-normalised bf16 batch instead of uint8 + fused preprocessing")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy (float32): the loss, and "
+                    "the updated parameters (step configs) or the parameter gradients (fwd+bwd configs), a fixed sample of up to 16384 entries per tensor")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes what the native step computed: it needs --impl native")
+    return args
 
 
 def peaks():
@@ -116,6 +125,21 @@ class ClockSampler:
             return None
         return {"sm_mhz": statistics.median(self.sm), "sm_max_mhz": self.max_sm, "reasons": sorted(self.reasons),
                 "power_w_max": max(self.power) if self.power else None, "samples": len(self.sm)}
+
+
+DUMP_PER_TENSOR = 16384       # at most 489 tensors (ViT-L) x 16384 x 4 B = 32 MB per dumped array
+
+
+def dump_sample(tensors):
+    """float32 concatenation, in the given order, of every tensor's entries, or of a fixed spread of DUMP_PER_TENSOR of them (a Weyl
+    sequence with a prime step over the flattened tensor) when it has more.  Runs on the device; returns a host array."""
+    out = []
+    for t in tensors:
+        f = t.detach().reshape(-1)
+        if f.numel() > DUMP_PER_TENSOR:
+            f = f[torch.arange(DUMP_PER_TENSOR, device=f.device) * 2654435761 % f.numel()]
+        out.append(f.float())
+    return torch.cat(out).cpu().numpy()
 
 
 def split3(B):
@@ -221,7 +245,7 @@ def run_reference(args, cfg, rank):
     if rank != 0:
         return
     b = cpu_sample_batch(cfg)
-    steps, warmup = min(args.steps, 10), min(args.warmup, 2)         # bounded: ~10-30 s of CPU work at ~1 s per step (c3; SURVEY 8d asks for >= 1 warm-up + 3 timed)
+    steps, warmup = args.steps, min(args.warmup, 2)          # ~1 s of CPU work per step (c3; SURVEY 8d asks for >= 1 warm-up + 3 timed)
     rate, threads, total = cpu_reference(cfg, steps, warmup, b)
     ms = 1000.0 * b / rate
     what = "fwd+bwd+clip+AdamW" if cfg["mode"] == "step" else "fwd+bwd"
@@ -428,6 +452,13 @@ def main():
     ms_step = t.item() / args.steps
     value = world * B / (ms_step / 1e3)
     final_loss = float(loss.item())
+    dump = None
+    if args.dump_outputs and rank == 0:          # read now: the passes below advance (end to end) and then garble (GEMM share) the state
+        if cfg["mode"] == "step":
+            dump = {"loss": loss, "params": [p for _, p in model.named_parameters()]}
+        else:
+            dump = {"loss": loss, "grads": [runner.G.views[n] for n in runner.G.names]}
+        dump = {k: dump_sample(v if isinstance(v, list) else [v]) for k, v in dump.items()}
 
     # ---- end to end: pinned host uint8 streams -> device -> step -> loss back on the host, every step
     for _ in range(2):
@@ -509,6 +540,11 @@ def main():
             except Exception as ex:      # the baseline is informative; never lose the GPU line to it
                 line["cpu_baseline"] = {"error": repr(ex)}
         print(json.dumps(line), flush=True)
+    if dump is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if world > 1:
         dist.destroy_process_group()
 

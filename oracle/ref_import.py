@@ -1,6 +1,7 @@
 """Import the UNMODIFIED reference backbone module for oracle pinning.  TEST INFRASTRUCTURE ONLY.
 
-Works only where ``/root/reference`` is mounted (the build container).  The reference file needs three
+Used by tests/golden/make_golden.py, which takes the root of a checkout of the original project (``--reference DIR``) and
+stores what the tests compare against under tests/golden/; the tests themselves never import it.  The reference file needs three
 ``timm`` helpers and one ``mmengine`` helper that are not installed; tiny shims with the documented
 semantics (timm 0.9.x ``drop_path``/``to_2tuple``/``trunc_normal_``; ``get_dist_info`` -> (0, 1)) are put
 into ``sys.modules`` before ``importlib`` executes the file where it lies (SURVEY.md Appendix D).
@@ -14,11 +15,7 @@ import types
 
 import torch
 
-REF_FILE = "/root/reference/Multi-Task_Pretrain/backbone/vit_win_rvsa_v3_wsz7.py"
-
-
-def reference_available() -> bool:
-    return os.path.isfile(REF_FILE)
+REF_FILE = "Multi-Task_Pretrain/backbone/vit_win_rvsa_v3_wsz7.py"      # relative to the root of the original project
 
 
 # When a test wants a deterministic train-mode comparison it fills this queue with per-call (B,) multipliers
@@ -38,9 +35,10 @@ def _drop_path(x, drop_prob: float = 0.0, training: bool = False, scale_by_keep:
     return x * r
 
 
-def load_reference_module():
-    if not reference_available():
-        raise FileNotFoundError(REF_FILE)
+def load_reference_module(root):
+    path = os.path.join(root, REF_FILE)
+    if not os.path.isfile(path):
+        raise FileNotFoundError(path)
     if "ref_rvsa" in sys.modules:
         return sys.modules["ref_rvsa"]
     tl = types.ModuleType("timm.models.layers")
@@ -52,7 +50,7 @@ def load_reference_module():
     for name, mod in (("timm", types.ModuleType("timm")), ("timm.models", types.ModuleType("timm.models")),
                       ("timm.models.layers", tl), ("mmengine", types.ModuleType("mmengine")), ("mmengine.dist", md)):
         sys.modules.setdefault(name, mod)
-    spec = importlib.util.spec_from_file_location("ref_rvsa", REF_FILE)
+    spec = importlib.util.spec_from_file_location("ref_rvsa", path)
     ref = importlib.util.module_from_spec(spec)
     import contextlib
     import io
@@ -62,12 +60,12 @@ def load_reference_module():
     return ref
 
 
-def build_reference(cfg_kwargs: dict, seed: int = 0):
+def build_reference(root, cfg_kwargs: dict, seed: int = 0):
     """Instantiate the reference class with ``cfg_kwargs`` and re-draw the zero-initialised rel-pos tables
     (they are ``zeros`` at init, [V]:83-84,216-217, which would leave the rel-pos terms untested)."""
     import contextlib
     import io
-    ref = load_reference_module()
+    ref = load_reference_module(root)
     torch.manual_seed(seed)
     with contextlib.redirect_stdout(io.StringIO()):
         model = ref.ViT_Win_RVSA_V3_WSZ7(**cfg_kwargs)

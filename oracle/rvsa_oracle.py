@@ -8,10 +8,9 @@ legs may import it.  The product path (``mtp_b200``) never does, and fails loudl
 library is missing.
 
 Pinning: the reference ships no tests or golden vectors for this path (SURVEY.md §4), so the oracle
-is pinned against the *live* reference module, imported unmodified in the build container
-(``oracle/ref_import.py``): ``tests/test_oracle_vs_reference.py`` (runs where ``/root/reference``
-exists) and the committed fixtures under ``tests/golden/`` (generated from the live reference by
-``tests/golden/make_golden.py``) which travel to the GPU box.
+is pinned against the *live* reference module, imported unmodified (``oracle/ref_import.py``) by
+``tests/golden/make_golden.py``, which stores the reference's results under ``tests/golden/``;
+``tests/test_oracle_vs_reference.py`` and ``tests/test_oracle_golden.py`` compare the oracle with them.
 
 All functions take the reference's ``state_dict`` key layout ([V] module tree, SURVEY.md §8b).
 """

@@ -1,7 +1,9 @@
 """Shared test utilities: golden fixture loading and oracle plumbing (tests only)."""
 import dataclasses
+import hashlib
 import os
 import statistics
+import zlib
 
 import numpy as np
 import torch
@@ -9,6 +11,85 @@ import torch
 from oracle import rvsa_oracle as O
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+MAP_SAMPLES = 512        # output-map entries kept per map in reference_pinning.npz
+TINY_MAP_SAMPLES = 4096  # ... and in tiny160.npz / tiny224.npz, whose sampled rel-L2 the GPU parity tests bound
+
+
+# ---- hashed test data: weights and inputs are a pure function of (seed, name, position) computed in integer arithmetic, so the fixtures
+#      taken from the original project need not store them and every machine regenerates them bit for bit
+def hash_uniform(n, seed):
+    """n float32 values in [0, 1): splitmix64 of (seed, index), top 24 bits."""
+    z = np.arange(n, dtype=np.uint64) + np.array([seed], dtype=np.uint64) * np.uint64(0x9E3779B97F4A7C15)
+    z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+    z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+    z = z ^ (z >> np.uint64(31))
+    return (z >> np.uint64(40)).astype(np.float32) / np.float32(2 ** 24)
+
+
+def hashed_tensor(shape, seed, name, std=1.0, mean=0.0):
+    """Uniform values of the given standard deviation and mean."""
+    u = hash_uniform(int(np.prod(shape)), (seed << 32) | zlib.crc32(name.encode()))
+    return torch.from_numpy((u * np.float32(2) - np.float32(1)) * np.float32(std * 3 ** 0.5) + np.float32(mean)).reshape(shape)
+
+
+def hashed_state_dict(template, seed):
+    """Weights for every floating-point entry of ``template`` (any state_dict of the backbone), at the scales of the reference's
+    initialisation: LayerNorm scales 1 +- 0.02, sampling heads ~ 4x a default Conv2d init, everything else std 0.02.  Integer
+    buffers are taken from ``template``."""
+    C = template["pos_embed"].shape[-1]
+    out = {}
+    for k, v in template.items():
+        if not v.is_floating_point():
+            out[k] = v.clone()
+        elif k.endswith(".weight") and v.ndim == 1:
+            out[k] = hashed_tensor(v.shape, seed, k, 0.02, 1.0)
+        else:
+            out[k] = hashed_tensor(v.shape, seed, k, 4.0 / (3 * C) ** 0.5 if ".sampling_" in k else 0.02)
+    return out
+
+
+def sample_points(n, k=MAP_SAMPLES):
+    """k distinct, evenly scattered flat indices into n entries (a Weyl sequence with a prime step)."""
+    return torch.from_numpy(((np.arange(min(n, k), dtype=np.uint64) * np.uint64(2654435761)) % np.uint64(n)).astype(np.int64))
+
+
+def map_summary(o, k=MAP_SAMPLES):
+    """What the fixtures keep of an output map: its shape, k entries (sample_points) and its per-channel means (float64)."""
+    return {"shape": np.array(o.shape, dtype=np.int64), "samples": o.reshape(-1)[sample_points(o.numel(), k)].numpy(),
+            "chmean": o.double().transpose(0, 1).reshape(o.shape[1], -1).mean(1).numpy()}
+
+
+def _map_refs(z, prefix, n_outs):
+    assert n_outs == sum(1 for k in z.files if k.startswith(prefix + "/out") and k.endswith("/shape"))
+    return [{f: z[f"{prefix}/out{i}/{f}"] for f in ("shape", "samples", "chmean")} for i in range(n_outs)]
+
+
+def check_maps(outs, z, prefix, tol):
+    """Every sampled entry and every channel mean of ``outs`` within ``tol`` of the stored reference values."""
+    for i, (o, ref) in enumerate(zip(outs, _map_refs(z, prefix, len(outs)))):
+        o = o.detach().cpu()
+        assert tuple(o.shape) == tuple(ref["shape"]), (prefix, i, tuple(o.shape))
+        got = map_summary(o, len(ref["samples"]))
+        assert float(np.abs(got["samples"] - ref["samples"]).max()) < tol, (prefix, i)
+        assert float(np.abs(got["chmean"] - ref["chmean"]).max()) < tol, (prefix, i)
+
+
+def sampled_rel_l2(outs, z, prefix):
+    """Per map: shape check, then the relative L2 distance of the stored sample of entries from the reference's."""
+    errs = []
+    for i, (o, ref) in enumerate(zip(outs, _map_refs(z, prefix, len(outs)))):
+        o = o.detach().float().cpu()
+        assert tuple(o.shape) == tuple(ref["shape"]), (prefix, i, tuple(o.shape))
+        got = o.reshape(-1)[sample_points(o.numel(), len(ref["samples"]))].double()
+        want = torch.from_numpy(ref["samples"]).double()
+        errs.append(float((got - want).norm() / want.norm().clamp_min(1e-30)))
+    return errs
+
+
+def tensor_sha256(t):
+    return hashlib.sha256(t.detach().contiguous().cpu().numpy().tobytes()).hexdigest()
+
+
 GOLDEN_CFGS = {
     "tiny160": dict(img_size=160, embed_dim=128, depth=4, num_heads=2, interval=2, out_indices=(0, 1, 2, 3)),
     "tiny224": dict(img_size=224, embed_dim=128, depth=4, num_heads=2, interval=2, out_indices=(0, 1, 2, 3)),
@@ -97,15 +178,44 @@ def parity_check(tag, m, outs, sd, cfg, x, keep, backward=True, direct=None):
     assert med <= GRAD_RATIO_MEDIAN, f"{tag}: median error ratio {med:.2f}"
 
 
+def golden_inputs(name, batch):
+    """The weights and the input the reference ran with for fixture ``name``: the reference's own initialisation under
+    torch.manual_seed(0), which the drop-in class reproduces bit for bit (tests/golden/make_golden.py checks it), with the re-draws
+    of oracle/ref_import.build_reference; the input is torch.randn under torch.manual_seed(1234).  The global RNG is left alone."""
+    from mtp_b200 import ViT_Win_RVSA_V3_WSZ7
+    c = GOLDEN_CFGS[name]
+    with torch.random.fork_rng(devices=[]):
+        torch.manual_seed(0)
+        m = ViT_Win_RVSA_V3_WSZ7(img_size=c["img_size"], patch_size=16, embed_dim=c["embed_dim"], depth=c["depth"], num_heads=c["num_heads"],
+                                 mlp_ratio=4, qkv_bias=True, use_abs_pos_emb=True, interval=c["interval"], out_indices=list(c["out_indices"]),
+                                 drop_path_rate=0.1, use_rel_pos_bias=True)
+        g = torch.Generator().manual_seed(1)
+        with torch.no_grad():
+            for n, p in m.named_parameters():
+                if "rel_pos" in n:
+                    p.copy_(torch.randn(p.shape, generator=g) * 0.02)
+                elif "sampling_" in n:
+                    p.mul_(4.0)
+                elif n.endswith(".bias") or "norm" in n or ".ln." in n:
+                    p.add_(torch.randn(p.shape, generator=g) * 0.02)
+        torch.manual_seed(1234)
+        x = torch.randn(batch, 3, c["img_size"], c["img_size"])
+    return {k: v.detach().clone() for k, v in m.state_dict().items()}, x
 
 
 def load_golden(name):
+    """Fixture ``name`` (tests/golden/make_golden.py): "sd" / "x" regenerated (golden_inputs, checked against the stored norms), the
+    reference's loss, its output maps as stored by map_summary ("z", prefix "fwd": check_maps / sampled_rel_l2) and its gradients
+    ("gnorm", "gfull", "gsamp")."""
     z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
-    g = {"x": torch.from_numpy(z["x"]), "loss": float(z["loss"]),
-         "outs": [torch.from_numpy(z[f"out{i}"]) for i in range(4)],
-         "sd": {}, "gnorm": {}, "gfull": {}, "gsamp": {}}
+    g = {"z": z, "loss": float(z["loss"]), "gnorm": {}, "gfull": {}, "gsamp": {}}
+    g["sd"], g["x"] = golden_inputs(name, int(z["batch"]))
+    for k, v in list(g["sd"].items()) + [("x", g["x"])]:
+        want = float(z["norm/" + k])
+        assert abs(float(v.double().norm()) - want) <= 1e-6 * max(want, 1.0), \
+            f"{name}: regenerated {k} is not what the reference ran with: the initialisation changed, regenerate the fixture"
     for k in z.files:
-        for grp in ("sd", "gnorm", "gfull", "gsamp"):
+        for grp in ("gnorm", "gfull", "gsamp"):
             if k.startswith(grp + "/"):
                 v = z[k]
                 g[grp][k[len(grp) + 1:]] = torch.from_numpy(v) if v.ndim else float(v)

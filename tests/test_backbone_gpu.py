@@ -3,7 +3,7 @@ import pytest
 import torch
 
 from oracle import rvsa_oracle as O
-from tests.helpers import GOLDEN_CFGS, load_golden, rel_l2
+from tests.helpers import GOLDEN_CFGS, load_golden, rel_l2, sampled_rel_l2
 
 pytestmark = pytest.mark.gpu
 
@@ -31,13 +31,17 @@ def test_forward_matches_golden(name, dtype):
     with torch.no_grad():
         outs = m(g["x"].cuda().to(dtype))
     assert isinstance(outs, list) and len(outs) == 4
-    errs = []
-    for o, r in zip(outs, g["outs"]):
-        assert o.shape == r.shape and o.dtype == dtype and o.is_contiguous()
-        errs.append(rel_l2(o.float().cpu(), r))
-    print(name, dtype, "rel-L2 per map:", ["%.2e" % e for e in errs])
+    assert all(o.dtype == dtype and o.is_contiguous() for o in outs)
+    # the reference's maps are stored as a fixed sample of entries; every entry is compared with the fp32 oracle, which
+    # tests/test_oracle_vs_reference.py and tests/test_oracle_golden.py hold to the reference
+    errs = sampled_rel_l2(outs, g["z"], "fwd")
+    with torch.no_grad():
+        o32 = O.backbone_forward(g["sd"], g["cfg"], g["x"])
+    errs_full = [rel_l2(o.float().cpu(), r) for o, r in zip(outs, o32)]
+    print(name, dtype, "rel-L2 per map vs reference (sampled):", ["%.2e" % e for e in errs], "vs fp32 oracle (full):",
+          ["%.2e" % e for e in errs_full])
     tol = FWD_REL_L2 if dtype == torch.float32 else 1.5 * FWD_REL_L2
-    assert max(errs) < tol, errs
+    assert max(errs) < tol and max(errs_full) < tol, (errs, errs_full)
 
 
 def test_forward_is_deterministic_and_batch_independent():

@@ -1,6 +1,6 @@
-"""Drop-in boundary (CPU): constructor kwargs, state_dict layout, factories, registry, config files, init_weights."""
-import ast
-import glob
+"""Drop-in boundary (CPU): constructor kwargs, state_dict layout, factories, registry, config files, init_weights.  What the reference
+module and its fine-tuning configs showed is stored in tests/golden/reference_boundary.json (tests/golden/make_golden.py)."""
+import json
 import os
 import types
 
@@ -9,10 +9,10 @@ import torch
 
 import mtp_b200
 from mtp_b200 import checkpoint
-from oracle import ref_import
+from tests.helpers import GOLDEN_DIR, hashed_state_dict, tensor_sha256
 
-REF_FT = "/root/reference/RS_Tasks_Finetune"
-HAVE_REF = ref_import.reference_available()
+with open(os.path.join(GOLDEN_DIR, "reference_boundary.json")) as _f:
+    REF = json.load(_f)
 
 
 def _tiny(**kw):
@@ -50,70 +50,43 @@ def test_layer_decay_names_are_parseable():
     assert all(layer_decay_group(n, tuple(p.shape), 6, "encoder.")[0] == 5 for n, p in m.named_parameters())
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference not mounted")
 @pytest.mark.parametrize("img", [160, 224])
 def test_state_dict_round_trip_with_reference(img):
-    ref = ref_import.build_reference(_tiny(img_size=img), seed=0)
+    ref = REF["state_dict_layout"][str(img)]
     new = mtp_b200.ViT_Win_RVSA_V3_WSZ7(**_tiny(img_size=img))
-    rs, ns = ref.state_dict(), new.state_dict()
-    assert list(rs.keys()) == list(ns.keys())
-    for k in rs:
-        assert rs[k].shape == ns[k].shape and rs[k].dtype == ns[k].dtype, k
-    assert torch.equal(rs["blocks.0.attn.relative_position_index"], ns["blocks.0.attn.relative_position_index"])
-    new.load_state_dict(rs, strict=True)
-    ref.load_state_dict(new.state_dict(), strict=True)
-    assert [n for n, _ in ref.named_parameters()] == [n for n, _ in new.named_parameters()]
+    ns = new.state_dict()
+    assert [k for k, _, _ in ref["keys"]] == list(ns.keys())
+    for k, shape, dtype in ref["keys"]:
+        assert list(ns[k].shape) == shape and str(ns[k].dtype) == dtype, k
+    assert tensor_sha256(ns["blocks.0.attn.relative_position_index"]) == ref["relative_position_index_sha256"]
+    rs = {k: torch.zeros(shape, dtype=getattr(torch, dtype[len("torch."):])) for k, shape, dtype in ref["keys"]}
+    new.load_state_dict(rs, strict=True)                    # a state_dict of the reference's layout loads strictly
+    assert [n for n, _ in new.named_parameters()] == ref["parameters"]
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference not mounted")
 def test_init_statistics_match_reference():
     """Same init recipe ([V]:676-691): trunc-normal(.02) linears, proj/fc2 rescaled by 1/sqrt(2*layer_id), LN = (1, 0)."""
-    ref = ref_import.load_reference_module()
-    import contextlib, io
-    torch.manual_seed(0)
-    with contextlib.redirect_stdout(io.StringIO()):
-        r = ref.ViT_Win_RVSA_V3_WSZ7(**_tiny())
     torch.manual_seed(0)
     n = mtp_b200.ViT_Win_RVSA_V3_WSZ7(**_tiny())
-    for k in ("blocks.0.attn.qkv.weight", "blocks.3.attn.proj.weight", "blocks.3.mlp.fc2.weight", "pos_embed"):
-        a, b = r.state_dict()[k], n.state_dict()[k]
-        assert abs(a.std().item() - b.std().item()) < 0.1 * a.std().item(), k
+    for k, ref_std in REF["init_std"].items():
+        assert abs(ref_std - n.state_dict()[k].std().item()) < 0.1 * ref_std, k
     assert float(n.blocks[1].norm1.weight.min()) == 1.0 and float(n.blocks[1].norm1.bias.abs().max()) == 0.0
     assert float(n.blocks[0].attn.rel_pos_h.abs().max()) == 0.0            # zero-initialised tables ([V]:216-217)
 
 
-def _backbone_dicts(path):
-    """Extract every `backbone=dict(...)` from a config file without importing mmengine."""
-    tree = ast.parse(open(path).read())
-    out = []
-    for node in ast.walk(tree):
-        if isinstance(node, ast.keyword) and node.arg == "backbone" and isinstance(node.value, ast.Call):
-            try:
-                out.append({kw.arg: ast.literal_eval(kw.value) for kw in node.value.keywords})
-            except Exception:
-                pass
-    return out
-
-
-@pytest.mark.skipif(not os.path.isdir(REF_FT), reason="/root/reference not mounted")
 def test_every_finetune_config_builds():
     """Every RS_Tasks_Finetune/**/configs/mtp/**/*rvsa*.py backbone dict constructs the matching twin (meta device)."""
-    files = sorted(glob.glob(os.path.join(REF_FT, "**", "configs", "mtp", "**", "*rvsa*.py"), recursive=True))
-    assert len(files) >= 60
+    ft = REF["finetune_configs"]
+    assert len(ft["files"]) >= 60
     built = 0
-    for f in files:
-        tk = ("mmseg" if "Semantic_Segmentation" in f else "mmpretrain" if "Scene_Classification" in f else
-              "opencd" if "Change_Detection" in f else "mmdet" if "Horizontal_Detection" in f else "mmrotate")
-        for cfg in _backbone_dicts(f):
-            if not str(cfg.get("type", "")).startswith("RVSA_MTP"):
-                continue
-            cfg = dict(cfg)
-            name = cfg.pop("type")
-            cfg["type"] = f"{tk}.{name}"
-            with torch.device("meta"):
-                m = mtp_b200.MODELS.build(cfg)
-            assert m.embed_dim in (768, 1024) and m.patch_embed.patch_shape[0] == cfg["img_size"] // 16
-            built += 1
+    for entry in ft["backbones"]:
+        cfg = dict(entry["backbone"])
+        name = cfg.pop("type")
+        cfg["type"] = f"{entry['toolkit']}.{name}"
+        with torch.device("meta"):
+            m = mtp_b200.MODELS.build(cfg)
+        assert m.embed_dim in (768, 1024) and m.patch_embed.patch_shape[0] == cfg["img_size"] // 16
+        built += 1
     assert built >= 60
 
 
@@ -163,24 +136,18 @@ def test_convert_state_dict_prefixes_and_resize():
     assert torch.equal(out2["pos_embed"], pe[:, 1:])
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="/root/reference not mounted")
 def test_init_weights_matches_reference(tmp_path):
     """init_weights(path) on the new class == the reference's own init_weights on the same checkpoint ([V]:693-778)."""
-    src = ref_import.build_reference(_tiny(img_size=160), seed=3)
+    src = hashed_state_dict(mtp_b200.ViT_Win_RVSA_V3_WSZ7(**_tiny(img_size=160)).state_dict(), 3)
     # an MAE-style checkpoint: cls-token slot in pos_embed, no full-attention rel-pos tables (they are grid-size specific and
     # the pretrain-variant loader does not resize them: a size mismatch raises in the reference too)
-    sd = {"encoder." + k: v for k, v in src.state_dict().items() if "full_attn_rel_pos" not in k}
-    sd["encoder.pos_embed"] = torch.cat([torch.zeros(1, 1, 128), src.state_dict()["pos_embed"]], 1)
+    sd = {"encoder." + k: v for k, v in src.items() if "full_attn_rel_pos" not in k}
+    sd["encoder.pos_embed"] = torch.cat([torch.zeros(1, 1, 128), src["pos_embed"]], 1)
     path = str(tmp_path / "ckpt.pth")
     torch.save({"state_dict": sd}, path)
-    import contextlib, io
     for img in (160, 224):                                 # same grid (strip cls token) and 10x10 -> 14x14 bicubic resize
-        kw = _tiny(img_size=img)
-        ref = ref_import.build_reference(kw, seed=9)
-        new = mtp_b200.ViT_Win_RVSA_V3_WSZ7(**kw)
-        with contextlib.redirect_stdout(io.StringIO()):
-            ref.init_weights(path)
+        new = mtp_b200.ViT_Win_RVSA_V3_WSZ7(**_tiny(img_size=img))
         new.init_weights(path)
-        rs, ns = ref.state_dict(), new.state_dict()
-        for k in ("pos_embed", "blocks.0.attn.qkv.weight", "blocks.2.attn.rel_pos_h", "fpn1.0.weight", "blocks.0.attn.sampling_offsets.2.weight"):
-            assert torch.equal(rs[k], ns[k]), (img, k)
+        ns = new.state_dict()
+        for k, ref in REF["init_weights"][str(img)].items():
+            assert list(ns[k].shape) == ref["shape"] and tensor_sha256(ns[k]) == ref["sha256"], (img, k)

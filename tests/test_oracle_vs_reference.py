@@ -1,11 +1,19 @@
-"""Pin the oracle against the LIVE reference module.  Runs only where /root/reference is mounted (build container)."""
+"""Pin the oracle against the reference module: the reference's results on hashed weights and inputs are stored in
+tests/golden/reference_pinning.npz (tests/golden/make_golden.py, run against a checkout of the original project)."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
+import mtp_b200
 from oracle import rvsa_oracle as O
-from oracle import ref_import
+from tests.helpers import GOLDEN_DIR, check_grads_against_golden, check_maps, hashed_state_dict, hashed_tensor
 
-pytestmark = pytest.mark.skipif(not ref_import.reference_available(), reason="/root/reference not mounted")
+
+@pytest.fixture(scope="module")
+def z():
+    return np.load(os.path.join(GOLDEN_DIR, "reference_pinning.npz"))
 
 
 def _kw(img, C, depth, nH, interval, oi, dpr=0.1):
@@ -13,67 +21,53 @@ def _kw(img, C, depth, nH, interval, oi, dpr=0.1):
                 use_abs_pos_emb=True, interval=interval, out_indices=list(oi), drop_path_rate=dpr, use_rel_pos_bias=True)
 
 
-def test_config1_vit_b_224_forward():
+def _weights(kw, seed):
+    """The hashed weights the reference ran with (its state_dict layout equals the drop-in class's: tests/test_boundary_cpu.py)."""
+    return hashed_state_dict(mtp_b200.ViT_Win_RVSA_V3_WSZ7(**kw).state_dict(), seed)
+
+
+def test_config1_vit_b_224_forward(z):
     """BASELINE.json configs[0]: ViT-B backbone forward, 1x3x224x224 on CPU."""
-    m = ref_import.build_reference(_kw(224, 768, 12, 12, 3, (3, 5, 7, 11)), seed=0)
+    P = _weights(_kw(224, 768, 12, 12, 3, (3, 5, 7, 11)), seed=0)
     cfg = O.vit_b_config(224)
-    torch.manual_seed(0)
-    x = torch.randn(1, 3, 224, 224)
     with torch.no_grad():
-        r = m(x)
-        o = O.backbone_forward(m.state_dict(), cfg, x)
-    for a, b in zip(r, o):
-        assert a.shape == b.shape and float((a - b).abs().max()) < 1e-5
+        o = O.backbone_forward(P, cfg, hashed_tensor((1, 3, 224, 224), 0, "input"))
+    check_maps(o, z, "vitb224", 1e-5)
 
 
 @pytest.mark.parametrize("img", [160, 320, 512])        # pad cases Hp 10->14, 20->21, 32->35
-def test_padded_grids(img):
-    m = ref_import.build_reference(_kw(img, 128, 4, 2, 2, (0, 1, 2, 3)), seed=3)
+def test_padded_grids(z, img):
+    P = _weights(_kw(img, 128, 4, 2, 2, (0, 1, 2, 3)), seed=3)
     cfg = O.OracleConfig(img_size=img, embed_dim=128, depth=4, num_heads=2, interval=2, out_indices=(0, 1, 2, 3))
-    torch.manual_seed(0)
-    x = torch.randn(2, 3, img, img)
     with torch.no_grad():
-        r = m(x)
-        o = O.backbone_forward(m.state_dict(), cfg, x)
-    for a, b in zip(r, o):
-        assert float((a - b).abs().max()) < 2e-5
+        o = O.backbone_forward(P, cfg, hashed_tensor((2, 3, img, img), 0, "input"))
+    check_maps(o, z, f"padded{img}", 2e-5)
 
 
-def test_backward_all_params():
-    m = ref_import.build_reference(_kw(160, 128, 4, 2, 2, (0, 1, 2, 3)), seed=5)
+def test_backward_all_params(z):
+    sd = _weights(_kw(160, 128, 4, 2, 2, (0, 1, 2, 3)), seed=5)
     cfg = O.OracleConfig(img_size=160, embed_dim=128, depth=4, num_heads=2, interval=2, out_indices=(0, 1, 2, 3))
-    torch.manual_seed(0)
-    x = torch.randn(2, 3, 160, 160)
-    O.synthetic_loss(m(x)).backward()
-    P = {k: (v.detach().clone().requires_grad_(True) if v.is_floating_point() else v) for k, v in m.state_dict().items()}
-    O.synthetic_loss(O.backbone_forward(P, cfg, x)).backward()
-    for k, p in m.named_parameters():
-        if p.grad is None:
-            assert k.startswith("norm.")
-            continue
-        err = float((P[k].grad - p.grad).norm() / p.grad.norm().clamp_min(1e-20))
-        assert err < 2e-4, (k, err)
+    P = {k: (v.clone().requires_grad_(True) if v.is_floating_point() else v) for k, v in sd.items()}
+    loss = O.synthetic_loss(O.backbone_forward(P, cfg, hashed_tensor((2, 3, 160, 160), 0, "input")))
+    assert abs(loss.item() - float(z["backward/loss"])) < 1e-5
+    loss.backward()
+    nograd = [str(k) for k in z["backward/nograd"]]
+    assert all(k.startswith("norm.") for k in nograd)        # the reference's final norm never gets a gradient
+    g = {"gnorm": {}, "gfull": {}, "gsamp": {}}
+    for k in z.files:
+        grp, _, name = k[len("backward/"):].partition("/")
+        if k.startswith("backward/") and grp in g:
+            g[grp][name] = float(z[k]) if grp == "gnorm" else torch.from_numpy(z[k])
+    assert set(g["gnorm"]) | set(nograd) == {k for k, v in sd.items() if v.is_floating_point()}
+    check_grads_against_golden({k: v.grad for k, v in P.items() if v.is_floating_point()}, g, tol=2e-4)
 
 
-def test_drop_path_train_mode():
+def test_drop_path_train_mode(z):
     """timm drop_path semantics: x * bernoulli(keep)/keep per sample, separate draws for attn and MLP branches."""
     kw = _kw(160, 128, 4, 2, 2, (0, 1, 2, 3), dpr=0.5)
-    m = ref_import.build_reference(kw, seed=7).train()
+    P = _weights(kw, seed=7)
     cfg = O.OracleConfig(img_size=160, embed_dim=128, depth=4, num_heads=2, interval=2, out_indices=(0, 1, 2, 3))
-    B = 4
-    torch.manual_seed(0)
-    x = torch.randn(B, 3, 160, 160)
-    rates = [r.item() for r in torch.linspace(0, 0.5, 4)]
-    g = torch.Generator().manual_seed(11)
-    keep = torch.ones(4, 2, B)
-    for i, r in enumerate(rates):
-        if r > 0:
-            keep[i] = torch.bernoulli(torch.full((2, B), 1 - r), generator=g) / (1 - r)
-    # block 0 has drop_prob 0 -> nn.Identity, no shim call
-    ref_import.KEEP_QUEUE[:] = [keep[i, j] for i in range(1, 4) for j in range(2)]
+    keep = torch.from_numpy(z["droppath/keep"])          # (depth, 2, B): the multipliers the reference's drop_path applied
     with torch.no_grad():
-        r = m(x)
-        o = O.backbone_forward(m.state_dict(), cfg, x, keep=keep)
-    assert not ref_import.KEEP_QUEUE
-    for a, b in zip(r, o):
-        assert float((a - b).abs().max()) < 2e-5
+        o = O.backbone_forward(P, cfg, hashed_tensor((4, 3, 160, 160), 0, "input"), keep=keep)
+    check_maps(o, z, "droppath", 2e-5)
